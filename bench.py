@@ -5,6 +5,7 @@
     python bench.py --gpus 1 --steps 20 --warmup 5
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference algorithm on the host cores (CPU oracle), same metric
+    python bench.py --steps 20 --warmup 5 --dump-outputs DIR   # also write the last timed step's outputs to DIR/<name>.npy
 
 One JSON line on stdout (rank 0).  `value` = crops/s of the whole job with inputs resident in HBM (device-timed, max over
 ranks) in the PARITY-BACKED mode ("mixed": fp32-faithful 3-pass forward + single-pass fp16 backward; its B = 64 outputs are
@@ -24,6 +25,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -142,6 +144,34 @@ def aux_from_batch(b):
                 gt_trans_ratio=b["roi_trans_ratio"])
 
 
+DUMP_HEAD_ROWS = 1 << 16   # of the B*64*64 head pixels (69 channels each)
+DUMP_GRAD_ELEMS = 1 << 21  # of the ~35M entries of the flat gradient
+DUMP_MAX_BYTES = 64 << 20
+
+
+def train_step_outputs(last, flat_grad):
+    """What a train step hands its caller, as host arrays for --dump-outputs: the 8 losses (engine.LOSS_NAMES order), the decoded
+    poses, and a fixed sample (seed 0, same rows / entries every run) of the 69-channel head maps and of the flat gradient, with
+    the sampled row / entry indices.  The full head and gradient (~210 MB) are sampled to stay under 64 MB."""
+    g = torch.Generator().manual_seed(0)
+    head = last["logits"].reshape(-1, 72)[:, :69]  # NHWC pixel rows: row = crop * 4096 + y * 64 + x
+    rows = torch.randperm(head.shape[0], generator=g)[:DUMP_HEAD_ROWS].sort().values
+    idx = torch.randperm(flat_grad.numel(), generator=g)[:DUMP_GRAD_ELEMS].sort().values
+    f32 = lambda t: t.detach().float().cpu().numpy()  # noqa: E731
+    return {"losses": f32(last["losses"]), "rot": f32(last["rot"]), "trans": f32(last["trans"]),
+            "head_sample": f32(head[rows.to(head.device)]), "head_sample_rows": rows.double().numpy(),
+            "grad_sample": f32(flat_grad[idx.to(flat_grad.device)]), "grad_sample_index": idx.double().numpy()}
+
+
+def dump_outputs(out_dir, arrays):
+    """DIR/<name>.npy per array (float32 / float64 only)."""
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_MAX_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     global BATCH_PER_GPU, WITH_SYM, METRIC
     if args.config == "ycbv":
@@ -162,10 +192,17 @@ def run_ours(args):
         dist.init_process_group("nccl", device_id=dev)
     B = BATCH_PER_GPU
     peaks = load_peaks()
+    # --dump-outputs: the train steps use the engine's ordered two-stage reductions for the BatchNorm statistics and backward
+    # sums instead of fp32 atomics, so that with the same arguments a step computes the same outputs every run and two builds
+    # can be compared output for output (the atomics' ordering jitter, ~1e-7, is amplified by the network's ReLU / max-pool
+    # decisions to ~1e-4 in the head maps and ~2e-2 in the gradients).  It costs one extra read of every pre-BN tensor in
+    # forward, so without --dump-outputs the default (atomics) path is timed; the JSON records which one ran.
+    deterministic = args.dump_outputs is not None
 
-    def one_mode(precision, steps, warmup, with_clocks):
+    def one_mode(precision, steps, warmup, with_clocks, capture_outputs=False):
         model, _opt = build(precision)
         eng = model.engine
+        eng.deterministic = deterministic
         reducer = GradAllReducer(eng.flat_grad, eng.named_params) if world > 1 else None
         eng.grad_hook = reducer
         batch = device_batch(synth.make_batch(B, seed=100 + rank, with_sym=WITH_SYM), dev)
@@ -180,7 +217,7 @@ def run_ours(args):
             eng.backward(gl)
             if reducer is not None:
                 reducer.finish()
-            last.update(losses=res["losses"], logits=res["logits"])
+            last.update(losses=res["losses"], logits=res["logits"], rot=res["rot"], trans=res["trans"])
             return res["losses"]
 
         step = eager_step
@@ -191,7 +228,7 @@ def run_ours(args):
             # forward + losses + backward + (N > 1) the bucketed NCCL all-reduces on their side stream: ONE graph per step
             graphed = GraphedTrainStep(eng, x, aux, train_bn=True)
             step = graphed
-            last.update(losses=graphed.losses, logits=graphed.logits)
+            last.update(losses=graphed.losses, logits=graphed.logits, rot=graphed.rot, trans=graphed.trans)
 
         for _ in range(warmup):
             losses = step()
@@ -224,15 +261,19 @@ def run_ours(args):
             ms = float(t)
         assert torch.isfinite(losses).all(), "non-finite losses"
         step_losses, step_logits = last["losses"].clone(), last["logits"].clone()  # outputs of the last TIMED step
+        # taken before the launch-count step below, which recomputes the same buffers
+        outputs = train_step_outputs(last, eng.flat_grad) if capture_outputs else None
         if graphed is not None:  # launches inside a replayed graph are not seen by the library's host-side counter
             l1 = launch_count()
             eager_step()
             launches = launch_count() - l1
             torch.cuda.synchronize()
         return dict(model=model, eng=eng, ms=ms, launches=launches, clocks=clocks, batch=batch, losses=step_losses,
-                    logits=step_logits, graphed=graphed is not None, precision=precision)
+                    logits=step_logits, graphed=graphed is not None, precision=precision, outputs=outputs)
 
-    main = one_mode(HEADLINE_MODE, args.steps, args.warmup, with_clocks=True)
+    main = one_mode(HEADLINE_MODE, args.steps, args.warmup, with_clocks=True, capture_outputs=bool(args.dump_outputs) and rank == 0)
+    if main["outputs"] is not None:
+        dump_outputs(args.dump_outputs, main.pop("outputs"))
     ms = main["ms"]
     value = world * B / (ms / 1e3)
     mode_desc = {
@@ -257,7 +298,8 @@ def run_ours(args):
                    "global_batch": world * B, "parallelism": f"dp{world}",
                    "l2": "activations per step (>2 GB) exceed the 126 MB L2; no explicit flush",
                    "launch": "whole step (incl. the NCCL all-reduces at N>1) replayed as one CUDA graph" if main["graphed"] else "eager (one ctypes call per kernel)",
-                   "grad_exchange": "bucketed NCCL all-reduce (AVG) of the flat 140 MB fp32 gradient buffer on a side stream, overlapped with backward, captured in the step graph" if world > 1 else "none"},
+                   "grad_exchange": "bucketed NCCL all-reduce (AVG) of the flat 140 MB fp32 gradient buffer on a side stream, overlapped with backward, captured in the step graph" if world > 1 else "none",
+                   "deterministic": deterministic},
         "clocks": main["clocks"], "gpu_launches": int(main["launches"]),
     }
 
@@ -318,7 +360,7 @@ def run_ours(args):
             loss_ev[i_last & 1].synchronize()
             read_back.append(float(loss_host[i_last & 1]))
 
-        n_e2e = max(3, args.steps)
+        n_e2e = args.steps
         cur = upload()
         # >= 8 untimed steps: the first one captures the forward / backward graphs, the next few let the caching allocator reach
         # its steady state (the prefetched input tensors are held by record_stream for a step, so early steps still cudaMalloc)
@@ -369,7 +411,7 @@ def run_ours(args):
                     out["modes"][prec] = {"value": round(B / (ms / 1e3), 1), "unit": "crops/s", "ms_per_step": round(ms, 3), "headline": True}
                     continue
                 try:
-                    r = one_mode(prec, max(5, args.steps // 2), 3, with_clocks=False)
+                    r = one_mode(prec, args.steps, 3, with_clocks=False)
                     out["modes"][prec] = {"value": round(B / (r["ms"] / 1e3), 1), "unit": "crops/s", "ms_per_step": round(r["ms"], 3),
                                           "what": mode_desc[prec]}
                     del r
@@ -575,6 +617,7 @@ def run_pnp(args):
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1) / args.steps
+        rot, t = rot.cpu(), t.cpu()  # outputs of the last timed step (the graph's output buffers are reused below)
         clocks = sampler.stop() if sampler else None
         if world > 1:
             tt = torch.tensor([ms], device=dev)
@@ -582,7 +625,7 @@ def run_pnp(args):
             ms = float(tt)
         # e2e: host buffers in, host results out, every step
         e0.record()
-        n_e2e = max(3, args.steps // 4)
+        n_e2e = args.steps
         for _ in range(n_e2e):
             r_, t_ = net(coor_h.to(dev, non_blocking=True), reg_h.to(dev, non_blocking=True), ext_h.to(dev, non_blocking=True))
             r_host, t_host = r_.cpu(), t_.cpu()
@@ -593,11 +636,13 @@ def run_pnp(args):
             tt = torch.tensor([ms_e2e], device=dev)
             dist.all_reduce(tt, op=dist.ReduceOp.MAX)
             ms_e2e = float(tt)
-        results[precision] = dict(ms=ms, ms_e2e=ms_e2e, rot=rot.cpu(), t=t.cpu(), clocks=clocks)
+        results[precision] = dict(ms=ms, ms_e2e=ms_e2e, rot=rot, t=t, clocks=clocks)
     if rank != 0:
         finish_distributed(world)
         return
     main = results["fp32x3"]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"rot": main["rot"].float().numpy(), "t": main["t"].float().numpy()})
     # algorithmic work (SURVEY 8d config 4): Conv / Linear MACs x 2 with the true nIn; bytes = fp32 input maps + fp32 weights
     flops = 2.0 * B * (1024 * 128 * 9 * nin + 256 * 128 * 9 * 128 + 64 * 128 * 9 * 128 + 8192 * 1024 + 1024 * 256 + 256 * 9)
     wbytes = 4.0 * sum(p.numel() for p in net.parameters())
@@ -833,7 +878,7 @@ def run_reference(args):
         o = O.gdrn_forward(leaf, batch, train=True, do_loss=True)
         sum(o["losses"].values()).backward()
 
-    steps, warm = max(1, min(args.steps, 5)), max(1, min(args.warmup, 2))
+    steps, warm = args.steps, max(1, min(args.warmup, 2))
     for _ in range(warm):
         step()
     t0 = time.perf_counter()
@@ -866,7 +911,14 @@ def main():
     ap.add_argument("--nin", type=int, default=69, choices=[67, 69], help="--config pnp: Patch-PnP input channels")
     ap.add_argument("--quick", action="store_true", help="device-timed value only (for profiler runs)")
     ap.add_argument("--no-graph", dest="graph", action="store_false", help="launch every kernel from Python instead of one CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0) to DIR/<name>.npy, float32/float64, at most 64 MB; "
+                         "the train steps then use ordered (run-to-run reproducible) reductions instead of fp32 atomics")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the CUDA arm's outputs; the reference arm times a CPU sample of the workload")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)

@@ -57,19 +57,39 @@ def test_unsupported_config_fails_loudly():
         G.build_model_optimizer(cfg)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/configs"), reason="reference tree only exists in the build container")
-def test_reference_config_files_load_and_match_builtin_a6():
-    ref = Config.fromfile("/root/reference/configs/gdrn/lm/a6_cPnP_lm13.py")
-    ref = postprocess_like_main_gdrn(ref, device="cpu")
+def test_reference_config_files_load_and_match_builtin_a6(golden_dir, tmp_path):
+    """The reference's a6_cPnP LM and YCB-V config files, as loaded (tests/golden/reference_configs.json, made by
+    oracle/make_golden_configs.py), set exactly the network that a6_config() builds.  The loader semantics those files rely on
+    (a `_base_` list whose base has a `_base_` string of its own, `_delete_` replacing an inherited dict) are checked on a
+    config chain of the same shape."""
+    import json
+
+    gold = json.load(open(os.path.join(golden_dir, "reference_configs.json")))
+    ref = postprocess_like_main_gdrn(Config(gold["lm13"]), device="cpu")
     ours = a6_config(device="cpu")
     r, o = ref.MODEL.CDPN.to_dict(), ours.MODEL.CDPN.to_dict()
     r["BACKBONE"]["PRETRAINED"] = ""
     assert r == o
     assert ref.SOLVER.BASE_LR == 1e-4 and ref.SOLVER.OPTIMIZER_CFG["type"] == "Ranger"
-    ycbv = Config.fromfile("/root/reference/configs/gdrn/ycbv/a6_cPnP_AugAAETrunc_BG0.5_Rsym_ycbv_real_pbr_visib20_10e.py")
+    ycbv = Config(gold["ycbv"])
     assert ycbv.MODEL.CDPN.PNP_NET.PM_LOSS_SYM is True
     # _delete_ semantics: OPTIMIZER_CFG replaced, not merged with the base's
     assert set(ref.SOLVER.OPTIMIZER_CFG.keys()) == {"type", "lr", "weight_decay"}
+
+    (tmp_path / "_base_").mkdir()
+    (tmp_path / "exp").mkdir()
+    (tmp_path / "_base_" / "common.py").write_text(
+        "SOLVER = dict(IMS_PER_BATCH=24, OPTIMIZER_CFG=dict(type='RMSprop', lr=1e-4, momentum=0.0, weight_decay=0))\n"
+        "MODEL = dict(CDPN=dict(NAME='GDRN', PNP_NET=dict(PM_LOSS_SYM=False, PM_LW=1.0)))\n")
+    (tmp_path / "_base_" / "model.py").write_text("_base_ = './common.py'\nMODEL = dict(CDPN=dict(TASK='rot'))\n")
+    (tmp_path / "exp" / "a6.py").write_text(
+        "_base_ = ['../_base_/model.py']\n"
+        "SOLVER = dict(OPTIMIZER_CFG=dict(_delete_=True, type='Ranger', lr=1e-4, weight_decay=0))\n"
+        "MODEL = dict(CDPN=dict(PNP_NET=dict(PM_LOSS_SYM=True)))\n")
+    cfg = postprocess_like_main_gdrn(Config.fromfile(str(tmp_path / "exp" / "a6.py")), device="cpu")
+    assert cfg.SOLVER.OPTIMIZER_CFG.to_dict() == {"type": "Ranger", "lr": 1e-4, "weight_decay": 0}
+    assert cfg.SOLVER.IMS_PER_BATCH == 24 and cfg.SOLVER.BASE_LR == 1e-4
+    assert cfg.MODEL.CDPN.to_dict() == {"NAME": "GDRN", "TASK": "rot", "PNP_NET": {"PM_LOSS_SYM": True, "PM_LW": 1.0}}
 
 
 def test_ranger_matches_reference_algorithm():

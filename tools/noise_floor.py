@@ -1,5 +1,5 @@
-import torch, sys
-sys.path.insert(0,'/root/repo')
+import os, torch, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from gdr_net_b200 import synth
 from oracle import fixtures, gdrn_oracle as O
 torch.set_num_threads(8)
